@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, bf16, batch 64 clips / GPU)
   python bench.py --impl reference --gpus N --steps K ...  # reference arm: CPU oracle port on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed forward computed, DIR/<name>.npy
 
 One "step" = one forward of SViT (configs/ssv2.yaml geometry, random init) over one batch of synthetic
 16x224^2 clips (BASELINE configs[1]).  `value` = clips/s with the batch resident in HBM; `e2e` = clips/s through the
@@ -132,7 +133,8 @@ def work_per_clip(cfg):
 
 # ------------------------------------------------------------------------------------------------ reference arm
 def cpu_forward_timing(max_seconds=25.0, max_runs=5):
-    """Times the CPU oracle port of the reference forward (fp32, batch 1, all host threads)."""
+    """Times the CPU oracle port of the reference forward (fp32, batch 1, all host threads).  Returns the run times, the
+    thread count and the (probs, extra) of the last run."""
     from oracle import svit_oracle as O
     from svit_b200.config import block_specs, ssv2_cfg, state_shapes
     from tests.golden.recipe import synth_input, synth_state
@@ -146,21 +148,47 @@ def cpu_forward_timing(max_seconds=25.0, max_runs=5):
     times = []
     t_begin = time.time()
     with torch.no_grad():
-        O.svit_forward(clip, params, specs, cfg)  # warm-up
+        out = O.svit_forward(clip, params, specs, cfg)  # warm-up
         while len(times) < max_runs and time.time() - t_begin < max_seconds:
             t0 = time.perf_counter()
-            O.svit_forward(clip, params, specs, cfg)
+            out = O.svit_forward(clip, params, specs, cfg)
             times.append(time.perf_counter() - t0)
-    return times, cores
+    return times, cores, out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def forward_outputs(probs, extra):
+    """What a caller of the forward receives, under the names --dump-outputs writes."""
+    d = {"forward_probs": probs}
+    d.update({f"forward_{k}": v for k, v in extra.items() if torch.is_tensor(v)})
+    return d
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as <path>/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all, each array is replaced by the
+    same fixed, seeded sample of its flattened elements, so two runs with the same arguments stay comparable element by
+    element."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(4 * v.numel() for v in arrays.values())
+    for name, v in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = v.numel() * DUMP_LIMIT_BYTES // total
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), v.numpy())
 
 
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, args.steps)
-    times, cores = cpu_forward_timing(max_seconds=120.0, max_runs=steps + args.warmup)
-    times = times[min(args.warmup, len(times) - 1):] or times
+    times, cores, (probs, extra) = cpu_forward_timing(max_seconds=float("inf"), max_runs=args.steps + args.warmup)
+    times = times[args.warmup:]
     sec = statistics.median(times)
     val = 1.0 / sec
     line = {"impl": "reference", "metric": "clips/sec (16x224^2, bf16) SViT forward", "value": val, "unit": "clips/s",
@@ -172,6 +200,8 @@ def run_reference(args):
                              "sample": f"{len(times)} batch-1 forwards of the oracle port (torch CPU fp32)"},
             "e2e": {"value": val, "unit": "clips/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, forward_outputs(probs, extra))
 
 
 # ------------------------------------------------------------------------------------------------ our arm
@@ -342,7 +372,17 @@ def main():
     ap.add_argument("--mode", default="both", choices=["both", "infer", "train"],
                     help="both: configs[1] headline + configs[2] as the 'train' object of the same JSON line; "
                          "train: only configs[2], printed as the main line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step of the timed forward legs (device-resident "
+                         "and end-to-end) computed as DIR/<name>.npy (float32, at most 64 MB in all); the inputs are "
+                         "seeded, so runs with the same arguments write the same arrays")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    # The training step is not a reproducible function of its inputs: its backward sums gradients with fp32 atomics in
+    # no fixed order, and the bf16 weight copies carry those last-bit differences into every later step.
+    if args.dump_outputs and args.mode == "train" and args.impl != "reference":
+        ap.error("--dump-outputs writes the forward legs' outputs; --mode train runs none")
     if args.impl == "reference":
         return run_reference(args)
     if args.mode == "train":
@@ -390,11 +430,14 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(K):
-            out, _ = model([dev_in[i & 1]] if args.no_graph else dev_in[i & 1])
+            out, extra = model([dev_in[i & 1]] if args.no_graph else dev_in[i & 1])
         e1.record()
         _barrier(world)
         ms = _max_over_ranks(e0.elapsed_time(e1), world, dev)
         launches = ops.launches() - l0
+        # copied now: the graph's static outputs are overwritten by the next replay
+        outputs = ({k: v.cpu() for k, v in forward_outputs(out, extra).items()}
+                   if args.dump_outputs and rank == 0 else None)
 
         # ---- end to end: pinned host clips -> H2D (copy stream, double buffered) -> forward -> D2H of the probabilities
         copy_stream = torch.cuda.Stream(device=dev)
@@ -438,6 +481,8 @@ def main():
         _barrier(world)
         ms_e2e = _max_over_ranks(s0.elapsed_time(s1), world, dev)
         clocks = sampler.stop() if rank == 0 else None
+        if outputs is not None:
+            outputs["e2e_probs"] = probs_host.clone()
 
         # ---- per-kernel breakdown (separate instrumented pass, CUDA events around every C-ABI call)
         prof = None
@@ -574,7 +619,7 @@ def main():
         except Exception as e:
             line["torch_gpu_baseline"] = {"unavailable": f"{type(e).__name__}: {str(e)[:160]}"}
     if world == 1 and not args.no_cpu_baseline:
-        times, cores = cpu_forward_timing(max_seconds=20.0, max_runs=5)
+        times, cores, _ = cpu_forward_timing(max_seconds=20.0, max_runs=5)
         sec = statistics.median(times)
         line["cpu_baseline"] = {"value": 1.0 / sec, "unit": "clips/s", "cores": cores, "kind": "port",
                                 "sample": f"{len(times)} batch-1 fp32 forwards of the CPU oracle port "
@@ -583,6 +628,8 @@ def main():
         with open(args.profile_json, "w") as f:
             json.dump(prof, f, indent=1)
     print(json.dumps(line), flush=True)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -1,8 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- loads the UNMODIFIED reference (eladb3/SViT) from /root/reference.
 
 Used only by tests/golden/make_golden.py (run in the build container, where the
-reference tree is mounted read-only) to produce the committed golden fixtures, and
-by CPU tests that cross-check the oracle restatement when the tree is present.
+reference tree is mounted read-only) to produce the committed golden fixtures.
 Nothing in svit_b200/ imports this file. /root/reference does not exist on the GPU box.
 
 Recipe (SURVEY.md 8c): the reference package cannot be imported as-is here because

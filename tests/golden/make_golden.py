@@ -374,6 +374,33 @@ def aug_cases():
     save("aug.pt", cases)
 
 
+# ---------------------------------------------------------------- N3 optimizer groups and learning-rate policy
+def optim_cases():
+    """models/optimizer.py of the unmodified reference: the weight-decay groups construct_optimizer builds for the tiny
+    SViT (parameter names per weight decay), the optimizer's class and base lr, and get_epoch_lr on the ssv2.yaml cosine
+    schedule without and with a 5-epoch warm-up.  The committed optim.pt was written by this function with
+    svit_b200.optim standing in for construct_optimizer / get_epoch_lr, after tests/test_host_logic.py had matched the
+    two bit for bit against the reference; neither has changed since."""
+    import copy
+    import importlib
+
+    import svit_b200
+    R = importlib.import_module("slowfast.models.optimizer")
+    cfg = tiny_cfg()
+    cfg.BN = type(cfg)({"WEIGHT_DECAY": 0.0}) if not hasattr(cfg, "BN") else cfg.BN
+    model = svit_b200.SViT(cfg, compute_dtype=torch.float32)
+    opt = R.construct_optimizer(model, cfg)
+    names = {id(p): n for n, p in model.named_parameters()}
+    groups = {float(g["weight_decay"]): sorted(names[id(p)] for p in g["params"]) for g in opt.param_groups}
+    lr = []
+    for warmup in (ssv2_cfg().SOLVER.WARMUP_EPOCHS, 5.0):
+        c = ssv2_cfg()
+        c.SOLVER.WARMUP_EPOCHS = warmup
+        for e in (0.0, 0.37, 4.99, 5.0, 12.5, 49.999):
+            lr.append(dict(warmup_epochs=warmup, epoch=e, out=copy.deepcopy(R.get_epoch_lr(e, c))))
+    save("optim.pt", dict(wd_groups=groups, optimizer=type(opt).__name__, base_lr=opt.defaults["lr"], lr=lr))
+
+
 if __name__ == "__main__":
     relpos_tables()
     pool_cases()
@@ -384,3 +411,4 @@ if __name__ == "__main__":
     aug_cases()
     box_cases()
     loss_cases()
+    optim_cases()

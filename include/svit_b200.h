@@ -229,6 +229,11 @@ int svit_assemble_tokens_bwd(const void* dx, float* dcls, float* dqueries, float
  * cols [B*To*Ho*Wo, Kpad], column order (c, kt, kh, kw), zero padded to Kpad. */
 int svit_im2col3d(const void* x, void* cols, int B, int Cin, int T, int H, int W, int kt, int kh, int kw, int st, int sh,
                   int sw, int pt, int ph, int pw, int Kpad, int in_dtype, int out_dtype, void* stream);
+/* Its transpose, the stem's data gradient on the CUDA cores: x [B, Cin, T, H, W] (out_dtype, overwritten) = for every input
+ * element the sum of the cols entries (in_dtype, same layout) of the <= ceil(kt/st) ceil(kh/sh) ceil(kw/sw) windows that
+ * read it.  Deterministic (a fixed summation order, no atomics). */
+int svit_col2im3d(const void* cols, void* x, int B, int Cin, int T, int H, int W, int kt, int kh, int kw, int st, int sh,
+                  int sw, int pt, int ph, int pw, int Kpad, int in_dtype, int out_dtype, void* stream);
 
 /* ---- PatchEmbed as an implicit GEMM (stem_helper.py:309-320; csrc/patch_embed_tc.cu): no im2col matrix.
  * svit_s2d_clip: the clip in space-to-depth cells, bf16 [B, ceil(T/st), ceil(H/sh), ceil(W/sw), C*st*sh*sw] with
@@ -243,6 +248,19 @@ int svit_patch_embed_s2d_supported(int C, int kt, int kh, int kw, int st, int sh
 int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, void* out, int64_t out_batch_stride,
                          int row_off, int B, int C, int T, int H, int W, int kt, int kh, int kw, int st, int sh, int sw,
                          int pt, int ph, int pw, int E, void* stream);
+/* Gradients with respect to the clip.  svit_patch_embed_s2d_dgrad: the transposed stem convolution on the same tensor-core
+ * kernel, dcells [B, ceil(T/st), ceil(H/sh), ceil(W/sw), C*st*sh*sw] bf16 (overwritten) from the patch rows of the bf16
+ * sequence gradient, read in place (row row_off + (t'*Ho + h')*Wo + w' of sample b at dy + b*dy_batch_stride, E values).
+ * w2t [C*st*sh*sw, ntaps*E] bf16 = the svit_patch_embed_s2d weight transposed with the tap order reversed in every
+ * dimension: w2t[cell, ((it*nh + ih)*nw + iw)*E + e] = w2[e, (((nt-1-it)*nh + nh-1-ih)*nw + nw-1-iw)*cell + cell].
+ * svit_patch_embed_s2d_dgrad_supported tells whether a geometry fits.  svit_d2s_clip: the inverse of svit_s2d_clip's cell
+ * layout, cells (bf16) -> x [B, C, T, H, W] in out_dtype (SVIT_F32 / SVIT_BF16); cell values beyond T/H/W are dropped. */
+int svit_patch_embed_s2d_dgrad_supported(int C, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph, int pw, int E);
+int svit_patch_embed_s2d_dgrad(const void* dy, int64_t dy_batch_stride, int row_off, const void* w2t, void* dcells, int B,
+                               int C, int T, int H, int W, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph,
+                               int pw, int E, void* stream);
+int svit_d2s_clip(const void* cells, void* x, int B, int C, int T, int H, int W, int st, int sh, int sw, int out_dtype,
+                  void* stream);
 
 /* ---- token split: video_model_builder.py:377-384. out [B, 1+O, C] = rows {0} U {N-O .. N-1} of x [B, N, C]. */
 int svit_gather_cls_obj_fwd(const void* x, void* out, int B, int64_t N, int O, int C, int dtype, void* stream);

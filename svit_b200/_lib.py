@@ -78,6 +78,7 @@ PROTOTYPES = {
     "svit_assemble_tokens_fwd": [vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp],
     "svit_assemble_tokens_bwd": [vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp],
     "svit_im2col3d": [vp, vp] + [C.c_int] * 17 + [vp],
+    "svit_col2im3d": [vp, vp] + [C.c_int] * 17 + [vp],
     "svit_gather_cls_obj_fwd": [vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int, vp],
     "svit_gather_cls_obj_bwd": [vp, vp, C.c_int, i64, C.c_int, C.c_int, C.c_int, vp],
     "svit_roi_tokens_fwd": [vp, i64, vp, vp, i64, vp, C.c_int, vp] + [C.c_int] * 8 + [f32, C.c_int, C.c_int, vp],
@@ -89,6 +90,9 @@ PROTOTYPES = {
     "svit_s2d_clip": [vp, vp] + [C.c_int] * 9 + [f32] * 6 + [vp],
     "svit_patch_embed_s2d_supported": [C.c_int] * 11,
     "svit_patch_embed_s2d": [vp, vp, vp, vp, i64, C.c_int] + [C.c_int] * 15 + [vp],
+    "svit_patch_embed_s2d_dgrad_supported": [C.c_int] * 11,
+    "svit_patch_embed_s2d_dgrad": [vp, i64, C.c_int, vp, vp] + [C.c_int] * 15 + [vp],
+    "svit_d2s_clip": [vp, vp] + [C.c_int] * 9 + [vp],
     "svit_crop_flip_normalize_u8": [vp, vp, vp, vp, vp] + [C.c_int] * 6 + [f32] * 6 + [C.c_int, vp],
     "svit_boxes_crop_flip": [vp, vp, vp, vp, vp, C.c_int, i64, C.c_int, C.c_int, f32, vp],
     "svit_head_fwd": [vp] * 14 + [C.c_int] * 8 + [vp],

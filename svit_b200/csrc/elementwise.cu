@@ -438,6 +438,40 @@ __global__ void im2col3d_kernel(const TI* __restrict__ x, TO* __restrict__ cols,
   }
 }
 
+// Transpose of im2col3d (the stem's data gradient on the CUDA cores): x[b, c, t, h, w] = the sum of cols[m, (c, dt, dh, dw)]
+// over the kernel taps whose output position m = ((t + pt - dt) / st, (h + ph - dh) / sh, (w + pw - dw) / sw) is whole and
+// in range.  One thread per input element sums its <= ceil(k / s)^3 windows in a fixed order: no atomics, deterministic.
+template <typename TI, typename TO>
+__global__ void col2im3d_kernel(const TI* __restrict__ cols, TO* __restrict__ x, int B, int Cin, int T_, int H, int W,
+                                int To, int Ho, int Wo, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph,
+                                int pw, int Kpad) {
+  const int64_t total = (int64_t)B * Cin * T_ * H * W;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int w = (int)(i % W), h = (int)((i / W) % H), t = (int)((i / ((int64_t)W * H)) % T_);
+    const int64_t bc = i / ((int64_t)W * H * T_);
+    const int c = (int)(bc % Cin), b = (int)(bc / Cin);
+    float acc = 0.f;
+    for (int dt = (t + pt) % st; dt < kt; dt += st) {
+      const int to = (t + pt - dt) / st;
+      if (to >= To) continue;
+      if (to < 0) break;
+      for (int dh = (h + ph) % sh; dh < kh; dh += sh) {
+        const int ho = (h + ph - dh) / sh;
+        if (ho >= Ho) continue;
+        if (ho < 0) break;
+        for (int dw = (w + pw) % sw; dw < kw; dw += sw) {
+          const int wo = (w + pw - dw) / sw;
+          if (wo >= Wo) continue;
+          if (wo < 0) break;
+          const int64_t m = (((int64_t)b * To + to) * Ho + ho) * Wo + wo;
+          acc += to_f(cols[m * Kpad + ((c * kt + dt) * kh + dh) * kw + dw]);
+        }
+      }
+    }
+    x[i] = from_f<TO>(acc);
+  }
+}
+
 // Generic dtype conversion / strided row gather used by the token split (video_model_builder.py:377-384):
 // out[b, j, :] = x[b, idx(j), :] for the rows {0} U {N-O..N-1}.
 template <typename T>
@@ -649,6 +683,27 @@ int svit_im2col3d(const void* x, void* cols, int B, int Cin, int T, int H, int W
   else if (in_dtype == SVIT_BF16 && out_dtype == SVIT_F32) IM2COL(bf16, float);
   else return SVIT_EINVAL;
 #undef IM2COL
+  SVIT_CHECK_LAUNCH();
+  return 0;
+}
+
+int svit_col2im3d(const void* cols, void* x, int B, int Cin, int T, int H, int W, int kt, int kh, int kw, int st_, int sh,
+                  int sw, int pt, int ph, int pw, int Kpad, int in_dtype, int out_dtype, void* stream) {
+  if (!cols || !x || B < 0 || Cin < 1 || T < 1 || H < 1 || W < 1 || st_ < 1 || sh < 1 || sw < 1 || pt < 0 || ph < 0 || pw < 0)
+    return SVIT_EINVAL;
+  int To = (T + 2 * pt - kt) / st_ + 1, Ho = (H + 2 * ph - kh) / sh + 1, Wo = (W + 2 * pw - kw) / sw + 1;
+  if (To < 1 || Ho < 1 || Wo < 1 || Kpad < Cin * kt * kh * kw) return SVIT_EINVAL;
+  int64_t total = (int64_t)B * Cin * T * H * W;
+  if (total == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  int g = grid_for(total, 256);
+#define COL2IM(TI, TO) col2im3d_kernel<TI, TO><<<g, 256, 0, st>>>((const TI*)cols, (TO*)x, B, Cin, T, H, W, To, Ho, Wo, kt, kh, kw, st_, sh, sw, pt, ph, pw, Kpad)
+  if (in_dtype == SVIT_F32 && out_dtype == SVIT_F32) COL2IM(float, float);
+  else if (in_dtype == SVIT_F32 && out_dtype == SVIT_BF16) COL2IM(float, bf16);
+  else if (in_dtype == SVIT_BF16 && out_dtype == SVIT_BF16) COL2IM(bf16, bf16);
+  else if (in_dtype == SVIT_BF16 && out_dtype == SVIT_F32) COL2IM(bf16, float);
+  else return SVIT_EINVAL;
+#undef COL2IM
   SVIT_CHECK_LAUNCH();
   return 0;
 }

@@ -405,6 +405,61 @@ __global__ void __launch_bounds__(256) s2d_rows_kernel(const void* __restrict__ 
   for (int i = threadIdx.x; i < g.Wc * cell / 8; i += blockDim.x) dst[i] = st4[i];
 }
 
+// Depth-to-space, the inverse of the cell layout (data gradient of svit_s2d_clip): x[b, c, t, h, w] = cells[b, t / st,
+// h / sh, w / sw, ((c st + t % st) sh + h % sh) sw + w % sw] for t < T, h < H, w < W (the rest of a partial cell is
+// dropped).  One CTA per row of cells (b, tc, hc): the row is read as one contiguous stream (into shared memory when it
+// fits 48 KB), then written as C st sh output rows, coalesced along w.  vec: sw == 4, W == 4 Wc, 16-byte aligned rows --
+// a thread moves one cell row (4 values).
+template <typename T>
+__global__ void __launch_bounds__(256) d2s_rows_kernel(const bf16* __restrict__ cells, T* __restrict__ x, S2dGeom g, int vec,
+                                                       int staged) {
+  extern __shared__ __align__(16) unsigned char d2s_smem[];
+  const int cell = g.C * g.st * g.sh * g.sw;
+  const int hc = blockIdx.x % g.Hc, tc_ = (blockIdx.x / g.Hc) % g.Tc, b = blockIdx.x / (g.Hc * g.Tc);
+  const bf16* src = cells + (((int64_t)b * g.Tc + tc_) * g.Hc + hc) * g.Wc * cell;
+  const bf16* rd = src;
+  if (staged) {
+    bf16* tile = reinterpret_cast<bf16*>(d2s_smem);  // [Wc][cell]
+    const int n = g.Wc * cell;
+    if (vec) {
+      for (int i = threadIdx.x; i < n / 8; i += blockDim.x)
+        reinterpret_cast<uint4*>(tile)[i] = __ldg(reinterpret_cast<const uint4*>(src) + i);
+    } else {
+      for (int i = threadIdx.x; i < n; i += blockDim.x) tile[i] = src[i];
+    }
+    __syncthreads();
+    rd = tile;
+  }
+  const int rows = g.C * g.st * g.sh;  // r = (c st + tt) sh + hh
+  if (vec) {
+    for (int i = threadIdx.x; i < rows * g.Wc; i += blockDim.x) {
+      const int wc = i % g.Wc, r = i / g.Wc;
+      const int hh = r % g.sh, tt = (r / g.sh) % g.st, c = r / (g.sh * g.st);
+      const int t = tc_ * g.st + tt, h = hc * g.sh + hh;
+      if (t >= g.T || h >= g.H) continue;
+      const uint2 v = *reinterpret_cast<const uint2*>(rd + wc * cell + r * 4);
+      const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.x));
+      const float2 c2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.y));
+      T* d = x + ((((int64_t)b * g.C + c) * g.T + t) * g.H + h) * g.W + (int64_t)wc * 4;
+      if constexpr (sizeof(T) == 4) {
+        *reinterpret_cast<float4*>(d) = make_float4(a.x, a.y, c2.x, c2.y);
+      } else {
+        *reinterpret_cast<uint2*>(d) = v;
+      }
+    }
+    return;
+  }
+  const int wmax = g.W;  // < Wc sw
+  for (int i = threadIdx.x; i < rows * wmax; i += blockDim.x) {
+    const int w = i % wmax, r = i / wmax;
+    const int hh = r % g.sh, tt = (r / g.sh) % g.st, c = r / (g.sh * g.st);
+    const int t = tc_ * g.st + tt, h = hc * g.sh + hh;
+    if (t >= g.T || h >= g.H) continue;
+    const int wc = w / g.sw;
+    x[((((int64_t)b * g.C + c) * g.T + t) * g.H + h) * g.W + w] = from_f<T>(__bfloat162float(rd[wc * cell + r * g.sw + (w - wc * g.sw)]));
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -448,39 +503,53 @@ int svit_s2d_clip(const void* x, void* cells, int B, int C, int T, int H, int W,
   return 0;
 }
 
-int svit_patch_embed_s2d_supported(int C, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph, int pw, int E) {
+
+int svit_d2s_clip(const void* cells, void* x, int B, int C, int T, int H, int W, int st, int sh, int sw, int out_dtype,
+                  void* stream) {
+  if (!cells || !x || B < 0 || C < 1 || T < 1 || H < 1 || W < 1 || st < 1 || sh < 1 || sw < 1) return SVIT_EINVAL;
+  if (out_dtype != SVIT_F32 && out_dtype != SVIT_BF16) return SVIT_EINVAL;
+  if (B == 0) return 0;
+  S2dGeom g{B, C, T, H, W, st, sh, sw, (T + st - 1) / st, (H + sh - 1) / sh, (W + sw - 1) / sw};
   const int cell = C * st * sh * sw;
-  if (cell % 32 || cell > 256 || E % 16 || E < 16 || E > PE_MAX_E) return 0;
-  auto taps = [](int k, int s, int p) {
-    auto fl = [](int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); };
-    return fl(k - 1 - p, s) - fl(-p, s) + 1;
-  };
-  const int ntaps = taps(kt, st, pt) * taps(kh, sh, ph) * taps(kw, sw, pw);
-  const int64_t w_bytes = (int64_t)ntaps * (cell / 32) * E * 64;
-  const int64_t smem = ((w_bytes + 1023) & ~1023) + (int64_t)PE_STAGES * (cell / 32) * PE_CHUNK_A + 2048 + 1024 + 256 + PE_MAX_E * 4;
-  return smem <= 227 * 1024 && (E == 96 || E == 128 || E == 192 || E == 256 || E == 64 || E == 32);
+  if ((int64_t)B * g.Tc * g.Hc >= (1ll << 31) || (int64_t)g.Wc * cell >= (1ll << 31)) return SVIT_ENOTSUP;
+  const bool aligned = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(cells) & 15) == 0;
+  const int vec = sw == 4 && W == 4 * g.Wc && ((int64_t)g.Wc * cell) % 8 == 0 && aligned;
+  const size_t tile = (size_t)g.Wc * cell * 2;
+  const int staged = tile <= 48 * 1024;
+  const unsigned grid = (unsigned)((int64_t)B * g.Tc * g.Hc);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (out_dtype == SVIT_F32)
+    d2s_rows_kernel<float><<<grid, 256, staged ? tile : 0, s>>>((const bf16*)cells, (float*)x, g, vec, staged);
+  else
+    d2s_rows_kernel<bf16><<<grid, 256, staged ? tile : 0, s>>>((const bf16*)cells, (bf16*)x, g, vec, staged);
+  SVIT_CHECK_LAUNCH();
+  return 0;
+}
+}  // extern "C"
+
+// First cell-tap offset (floor(-p / s)) and tap count of one dimension of a stride-s, padding-p, size-k convolution.
+static void pe_taps(int k, int s, int pad, int* lo, int* n) {
+  auto fl = [](int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); };
+  *lo = fl(-pad, s);
+  *n = fl(k - 1 - pad, s) - *lo + 1;
 }
 
-// cells [B, Tc, Hc, Wc, cell] bf16 (svit_s2d_clip); w2 [E, ntaps * cell] bf16 (zero-padded taps, tap-major:
-// ((it nh + ih) nw + iw) cell + inner); out rows row_off + (t' Ho + h') Wo + w' of every sample (out_batch_stride elements)
-int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, void* out, int64_t out_batch_stride,
-                         int row_off, int B, int C, int T, int H, int W, int kt, int kh, int kw, int st, int sh, int sw,
-                         int pt, int ph, int pw, int E, void* stream) {
-  if (!cells || !w2 || !out || B < 0) return SVIT_EINVAL;
-  if (!svit_patch_embed_s2d_supported(C, kt, kh, kw, st, sh, sw, pt, ph, pw, E)) return SVIT_ENOTSUP;
-  if ((reinterpret_cast<uintptr_t>(cells) | reinterpret_cast<uintptr_t>(w2) | reinterpret_cast<uintptr_t>(out)) & 15)
-    return SVIT_ENOTSUP;
-  if (B == 0) return 0;
-  auto fl = [](int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); };
-  PeParams p;
-  const int cell = C * st * sh * sw;
-  p.B = B; p.Tc = (T + st - 1) / st; p.Hc = (H + sh - 1) / sh; p.Wc = (W + sw - 1) / sw;
-  p.To = (T + 2 * pt - kt) / st + 1; p.Ho = (H + 2 * ph - kh) / sh + 1; p.Wo = (W + 2 * pw - kw) / sw + 1;
-  p.lo_t = fl(-pt, st); p.lo_h = fl(-ph, sh); p.lo_w = fl(-pw, sw);
-  p.nt = fl(kt - 1 - pt, st) - p.lo_t + 1; p.nh = fl(kh - 1 - ph, sh) - p.lo_h + 1; p.nw = fl(kw - 1 - pw, sw) - p.lo_w + 1;
+static int64_t pe_smem_bytes(int ntaps, int chunks, int n_cols, int stages, int chunk_a) {
+  return (((int64_t)ntaps * chunks * n_cols * 64 + 1023) & ~(int64_t)1023) + (int64_t)stages * chunks * chunk_a + 2048 + 1024 +
+         256 + PE_MAX_E * 4;
+}
+
+static bool pe_n_ok(int n) { return n == 32 || n == 64 || n == 96 || n == 128 || n == 192 || n == 256; }
+
+// One stride-1 implicit-GEMM convolution over a channels-last 5-D input `in` (dims {K1, Wi, Hi, Ti, B} innermost first,
+// byte strides of the outer four; K1 = p.chunks * 32 values per position) into rows row_off + (t Ho + h) Wo + w of
+// every sample of p.out (p.E values each).  p carries the output grid (To, Ho, Wo), the taps (nt, nh, nw) and their
+// first offsets (lo_*); w2 [p.E, ntaps * K1] bf16.  Used as the stem forward (in = cells, out = patch rows) and as its
+// data gradient (in = the patch rows of the sequence gradient, out = cell gradients).
+static int pe_launch(PeParams p, const void* in, const cuuint64_t in_dims[5], const cuuint64_t in_strides[4], const void* w2,
+                     cudaStream_t s) {
+  const int E = p.E;
   if (p.Wo < 1 || p.Wo > 128 || p.Ho < 1 || p.To < 1 || (E * 2) % 16) return SVIT_ENOTSUP;
-  p.chunks = cell / 32;
-  p.E = E;
   // SVIT_PE_MODE=0: one shifted TMA box per tap (every cell fetched up to 8 times from L2); 1 (default): every cell of the
   // tile's halo box once, the taps are row-shifted views of it -- the swizzle of a K-major tile is a function of the
   // absolute shared-memory address, so a descriptor whose start is shifted by whole rows (base offset 0) reads exactly the
@@ -498,26 +567,22 @@ int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, v
   p.PH = p.R + p.nh - 1;
   p.chunk_a = p.uniq ? ((p.PH * p.PW * 64 + 1023) & ~1023) : PE_CHUNK_A;
   p.tiles_h = (p.Ho + p.R - 1) / p.R;
-  p.tiles = (int64_t)B * p.To * p.tiles_h;
-  p.out_bs = out_batch_stride;
-  p.row_off = row_off;
-  p.bias = bias;
-  p.out = (bf16*)out;
+  p.tiles = (int64_t)p.B * p.To * p.tiles_h;
   p.w_chunk_bytes = E * 64;
   svit_tmap_encode_fn enc = svit_get_tmap_encode();
   if (!enc) return SVIT_ENOTSUP;
   CUtensorMap tx, tw;
   {
-    cuuint64_t dims[5] = {(cuuint64_t)cell, (cuuint64_t)p.Wc, (cuuint64_t)p.Hc, (cuuint64_t)p.Tc, (cuuint64_t)B};
-    cuuint64_t strides[4] = {(cuuint64_t)cell * 2, (cuuint64_t)p.Wc * cell * 2, (cuuint64_t)p.Hc * p.Wc * cell * 2,
-                             (cuuint64_t)p.Tc * p.Hc * p.Wc * cell * 2};
+    cuuint64_t dims[5], strides[4];
+    for (int i = 0; i < 5; ++i) dims[i] = in_dims[i];
+    for (int i = 0; i < 4; ++i) strides[i] = in_strides[i];
     cuuint32_t box[5] = {32, (cuuint32_t)(p.uniq ? p.PW : p.Wo), (cuuint32_t)(p.uniq ? p.PH : p.R), 1, 1};
     cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    if (enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(cells), dims, strides, box, estr,
+    if (enc(&tx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(in), dims, strides, box, estr,
             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
       return SVIT_EINVAL;
-    const int ktot = p.nt * p.nh * p.nw * cell;
+    const int ktot = p.nt * p.nh * p.nw * p.chunks * 32;
     cuuint64_t wd[2] = {(cuuint64_t)ktot, (cuuint64_t)E};
     cuuint64_t ws[1] = {(cuuint64_t)ktot * 2};
     cuuint32_t wb[2] = {32, (cuuint32_t)E};
@@ -527,12 +592,10 @@ int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, v
       return SVIT_EINVAL;
   }
   const int ntaps = p.nt * p.nh * p.nw;
-  const size_t smem = (((size_t)ntaps * p.chunks * p.w_chunk_bytes + 1023) & ~(size_t)1023) +
-                      (size_t)(p.uniq ? 2 : PE_STAGES) * p.chunks * p.chunk_a + 2048 + 1024 + 256 + PE_MAX_E * 4;
+  const size_t smem = (size_t)pe_smem_bytes(ntaps, p.chunks, E, p.uniq ? 2 : PE_STAGES, p.chunk_a);
   if (smem > 227 * 1024) return SVIT_ENOTSUP;
   int64_t grid = svit_num_sms();
   if (grid > p.tiles) grid = p.tiles;
-  cudaStream_t s = (cudaStream_t)stream;
 #define PE_LAUNCH(EV)                                                                                              \
   {                                                                                                                \
     auto kern = patch_embed_tc_kernel<EV>;                                                                         \
@@ -555,6 +618,96 @@ int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, v
 #undef PE_LAUNCH
   SVIT_CHECK_LAUNCH();
   return 0;
+}
+
+extern "C" {
+
+int svit_patch_embed_s2d_supported(int C, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph, int pw, int E) {
+  const int cell = C * st * sh * sw;
+  if (cell % 32 || cell > 256 || E % 16 || E < 16 || E > PE_MAX_E) return 0;
+  int lo, nt, nh, nw;
+  pe_taps(kt, st, pt, &lo, &nt);
+  pe_taps(kh, sh, ph, &lo, &nh);
+  pe_taps(kw, sw, pw, &lo, &nw);
+  return pe_smem_bytes(nt * nh * nw, cell / 32, E, PE_STAGES, PE_CHUNK_A) <= 227 * 1024 && pe_n_ok(E);
+}
+
+// cells [B, Tc, Hc, Wc, cell] bf16 (svit_s2d_clip); w2 [E, ntaps * cell] bf16 (zero-padded taps, tap-major:
+// ((it nh + ih) nw + iw) cell + inner); out rows row_off + (t' Ho + h') Wo + w' of every sample (out_batch_stride elements)
+int svit_patch_embed_s2d(const void* cells, const void* w2, const float* bias, void* out, int64_t out_batch_stride,
+                         int row_off, int B, int C, int T, int H, int W, int kt, int kh, int kw, int st, int sh, int sw,
+                         int pt, int ph, int pw, int E, void* stream) {
+  if (!cells || !w2 || !out || B < 0) return SVIT_EINVAL;
+  if (!svit_patch_embed_s2d_supported(C, kt, kh, kw, st, sh, sw, pt, ph, pw, E)) return SVIT_ENOTSUP;
+  if ((reinterpret_cast<uintptr_t>(cells) | reinterpret_cast<uintptr_t>(w2) | reinterpret_cast<uintptr_t>(out)) & 15)
+    return SVIT_ENOTSUP;
+  if (B == 0) return 0;
+  PeParams p;
+  const int cell = C * st * sh * sw;
+  p.B = B; p.Tc = (T + st - 1) / st; p.Hc = (H + sh - 1) / sh; p.Wc = (W + sw - 1) / sw;
+  p.To = (T + 2 * pt - kt) / st + 1; p.Ho = (H + 2 * ph - kh) / sh + 1; p.Wo = (W + 2 * pw - kw) / sw + 1;
+  pe_taps(kt, st, pt, &p.lo_t, &p.nt);
+  pe_taps(kh, sh, ph, &p.lo_h, &p.nh);
+  pe_taps(kw, sw, pw, &p.lo_w, &p.nw);
+  p.chunks = cell / 32;
+  p.E = E;
+  p.out_bs = out_batch_stride;
+  p.row_off = row_off;
+  p.bias = bias;
+  p.out = (bf16*)out;
+  const cuuint64_t dims[5] = {(cuuint64_t)cell, (cuuint64_t)p.Wc, (cuuint64_t)p.Hc, (cuuint64_t)p.Tc, (cuuint64_t)B};
+  const cuuint64_t strides[4] = {(cuuint64_t)cell * 2, (cuuint64_t)p.Wc * cell * 2, (cuuint64_t)p.Hc * p.Wc * cell * 2,
+                                 (cuuint64_t)p.Tc * p.Hc * p.Wc * cell * 2};
+  return pe_launch(p, cells, dims, strides, w2, (cudaStream_t)stream);
+}
+
+// Data gradient of the stem: the same kernel with the roles swapped.  Cell c of a dimension is read by the outputs
+// c - lo - i (i < n taps), so dcells[c] = sum_i' dY[c + lo' + i'] . W''_i' with lo' = -lo - n + 1 and W''_i' = W'_{n-1-i'}^T:
+// a stride-1 convolution over the output grid (K = E values per position) into the cell grid (N = cell values per cell).
+int svit_patch_embed_s2d_dgrad_supported(int C, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph, int pw, int E) {
+  const int cell = C * st * sh * sw;
+  if (E % 32 || E < 32 || E > PE_MAX_E || !pe_n_ok(cell)) return 0;
+  int lo, nt, nh, nw;
+  pe_taps(kt, st, pt, &lo, &nt);
+  pe_taps(kh, sh, ph, &lo, &nh);
+  pe_taps(kw, sw, pw, &lo, &nw);
+  return pe_smem_bytes(nt * nh * nw, E / 32, cell, PE_STAGES, PE_CHUNK_A) <= 227 * 1024;
+}
+
+// dy: sequence gradient, bf16, sample b's patch row (t' Ho + h') Wo + w' at dy + b dy_batch_stride + (row_off + ...) E,
+// read in place; w2t [cell, ntaps * E] bf16 (svit_b200.ops.s2d_dgrad_weight); dcells [B, Tc, Hc, Wc, cell] bf16.
+int svit_patch_embed_s2d_dgrad(const void* dy, int64_t dy_batch_stride, int row_off, const void* w2t, void* dcells, int B,
+                               int C, int T, int H, int W, int kt, int kh, int kw, int st, int sh, int sw, int pt, int ph,
+                               int pw, int E, void* stream) {
+  if (!dy || !w2t || !dcells || B < 0 || row_off < 0 || dy_batch_stride < 0) return SVIT_EINVAL;
+  if (!svit_patch_embed_s2d_dgrad_supported(C, kt, kh, kw, st, sh, sw, pt, ph, pw, E)) return SVIT_ENOTSUP;
+  const bf16* dy0 = (const bf16*)dy + (int64_t)row_off * E;
+  if ((reinterpret_cast<uintptr_t>(dy0) | reinterpret_cast<uintptr_t>(w2t) | reinterpret_cast<uintptr_t>(dcells)) & 15 ||
+      (dy_batch_stride * 2) % 16)
+    return SVIT_ENOTSUP;
+  if (B == 0) return 0;
+  const int cell = C * st * sh * sw;
+  const int To = (T + 2 * pt - kt) / st + 1, Ho = (H + 2 * ph - kh) / sh + 1, Wo = (W + 2 * pw - kw) / sw + 1;
+  if (To < 1 || Ho < 1 || Wo < 1) return SVIT_EINVAL;
+  if ((int64_t)To * Ho * Wo * E > dy_batch_stride && B > 1) return SVIT_EINVAL;
+  PeParams p;
+  p.B = B; p.Tc = (T + st - 1) / st; p.Hc = (H + sh - 1) / sh; p.Wc = (W + sw - 1) / sw;
+  p.To = p.Tc; p.Ho = p.Hc; p.Wo = p.Wc;  // the output grid is the cell grid
+  pe_taps(kt, st, pt, &p.lo_t, &p.nt);
+  pe_taps(kh, sh, ph, &p.lo_h, &p.nh);
+  pe_taps(kw, sw, pw, &p.lo_w, &p.nw);
+  p.lo_t = -p.lo_t - p.nt + 1; p.lo_h = -p.lo_h - p.nh + 1; p.lo_w = -p.lo_w - p.nw + 1;
+  p.chunks = E / 32;
+  p.E = cell;
+  p.out_bs = (int64_t)p.Tc * p.Hc * p.Wc * cell;
+  p.row_off = 0;
+  p.bias = nullptr;
+  p.out = (bf16*)dcells;
+  // dY positions outside the output grid are the TMA zero fill
+  const cuuint64_t dims[5] = {(cuuint64_t)E, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)To, (cuuint64_t)B};
+  const cuuint64_t strides[4] = {(cuuint64_t)E * 2, (cuuint64_t)Wo * E * 2, (cuuint64_t)Ho * Wo * E * 2,
+                                 (cuuint64_t)(B > 1 ? dy_batch_stride : (int64_t)To * Ho * Wo * E) * 2};
+  return pe_launch(p, dy0, dims, strides, w2t, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -98,7 +98,8 @@ _FAMILY = {"svit_gemm": "gemm", "svit_attn_fwd": "attention", "svit_attn_bwd": "
            "svit_pool_ln_fwd": "pool_ln", "svit_pool_ln_fwd_save": "pool_ln", "svit_pool_ln_bwd": "pool_ln_bwd",
            "svit_pool_ln_bwd_saved": "pool_ln_bwd", "svit_layernorm_fwd": "layernorm", "svit_row_stats": "layernorm",
            "svit_layernorm_bwd": "layernorm_bwd", "svit_skip_maxpool_fwd": "skip_pool", "svit_skip_maxpool_fwd_idx": "skip_pool", "svit_im2col3d": "im2col", "svit_s2d_clip": "im2col",
-           "svit_patch_embed_s2d": "gemm", "svit_mlp_fused": "gemm"}
+           "svit_patch_embed_s2d": "gemm", "svit_mlp_fused": "gemm",
+           "svit_patch_embed_s2d_dgrad": "gemm", "svit_d2s_clip": "im2col", "svit_col2im3d": "im2col"}
 _prof = None
 
 
@@ -860,30 +861,57 @@ class _PatchEmbedTokens(torch.autograd.Function):
         gemm(cols, w2, x, B * L, E, Kpad, Kpad, Kpad, E, 0, 1, bias=_f32(b), remap=(L, Ntot, 1))
         _call("svit_assemble_tokens_fwd", x.data_ptr(), _f32(cls).data_ptr(), _f32(queries).data_ptr(),
               _f32(pos_t).data_ptr(), B, L, Tx, O, E, odt, _stream())
-        ctx.save_for_backward(cols)
+        ctx.save_for_backward(cols if ctx.needs_input_grad[1] else None, w)
         ctx.geom = (B, L, Tx, O, E, K, Kpad, Ntot)
         ctx.shapes = (w.shape, cls.shape, queries.shape, pos_t.shape)
+        ctx.conv = (clip.shape, clip.dtype, tuple(kernel), tuple(stride), tuple(padding))
         return x
 
     @staticmethod
     def backward(ctx, dx):
-        (cols,) = ctx.saved_tensors
+        cols, w = ctx.saved_tensors
         B, L, Tx, O, E, K, Kpad, Ntot = ctx.geom
         wshape, cshape, qshape, pshape = ctx.shapes
+        need = ctx.needs_input_grad
         dx = dx.contiguous()
         dev = dx.device
-        # patch rows of dx as a strided [B*L, E] view are not contiguous across samples -> compact copy via gather GEMM
-        dpatch = dx[:, 1:1 + L].reshape(B * L, E)  # torch view/copy glue (autograd tape only)
-        dw = torch.empty(E, Kpad, dtype=torch.float32, device=dev)
-        gemm(dpatch, cols, dw, E, Kpad, B * L, E, Kpad, Kpad, 1, 0)
-        db = _colsum(dpatch, B * L, E)
-        dcls = torch.zeros(E, dtype=torch.float32, device=dev)
-        dq = torch.zeros(O * E, dtype=torch.float32, device=dev)
-        dp = torch.zeros(pshape[1] * E, dtype=torch.float32, device=dev)
-        _call("svit_assemble_tokens_bwd", dx.data_ptr(), dcls.data_ptr(), dq.data_ptr(), dp.data_ptr(), B, L, Tx, O, E,
-              _dt(dx), _stream())
-        return (None, dw[:, :K].reshape(wshape), db, dcls.reshape(cshape), dq.reshape(qshape), dp.reshape(pshape),
-                None, None, None, None)
+        dclip = dw = db = dcls = dq = dp = None
+        if need[0]:
+            dclip = patch_embed_input_grad(dx, w, *ctx.conv)
+        if need[1] or need[2]:
+            # patch rows of dx as a strided [B*L, E] view are not contiguous across samples -> compact copy via gather GEMM
+            dpatch = dx[:, 1:1 + L].reshape(B * L, E)  # torch view/copy glue (autograd tape only)
+            if need[1]:
+                dw = torch.empty(E, Kpad, dtype=torch.float32, device=dev)
+                gemm(dpatch, cols, dw, E, Kpad, B * L, E, Kpad, Kpad, 1, 0)
+                dw = dw[:, :K].reshape(wshape)
+            if need[2]:
+                db = _colsum(dpatch, B * L, E)
+        if any(need[3:6]):
+            dcls = torch.zeros(E, dtype=torch.float32, device=dev)
+            dq = torch.zeros(O * E, dtype=torch.float32, device=dev)
+            dp = torch.zeros(pshape[1] * E, dtype=torch.float32, device=dev)
+            _call("svit_assemble_tokens_bwd", dx.data_ptr(), dcls.data_ptr(), dq.data_ptr(), dp.data_ptr(), B, L, Tx, O, E,
+                  _dt(dx), _stream())
+            dcls, dq, dp = dcls.reshape(cshape), dq.reshape(qshape), dp.reshape(pshape)
+        return dclip, dw, db, dcls, dq, dp, None, None, None, None
+
+
+class _PatchEmbedInputGrad(torch.autograd.Function):
+    """The stem when only the clip needs a gradient (a frozen model: saliency, attribution, adversarial inputs): the
+    bf16 implicit-GEMM forward of inference, no im2col matrix saved, and a backward that runs the data gradient alone."""
+
+    @staticmethod
+    def forward(ctx, clip, w, b, cls, queries, pos_t, kernel, stride, padding):
+        x = _patch_embed_implicit(clip, w, b, cls, queries, pos_t, kernel, stride, padding, None, None)
+        ctx.save_for_backward(w)
+        ctx.conv = (clip.shape, clip.dtype, kernel, stride, padding)
+        return x
+
+    @staticmethod
+    def backward(ctx, dx):
+        (w,) = ctx.saved_tensors
+        return (patch_embed_input_grad(dx.contiguous(), w, *ctx.conv),) + (None,) * 8
 
 
 def _padded_weight(w, K, Kpad, dtype):
@@ -900,16 +928,14 @@ def _floor_div(a, b):
     return a // b  # Python floors towards -inf, which is what the tap arithmetic needs
 
 
-def s2d_conv_weight(w, stride, padding):
-    """Conv3d weight [E, C, kt, kh, kw] scattered into the space-to-depth taps of csrc/patch_embed_tc.cu:
-    W2[E, ((it*nh + ih)*nw + iw) * cell + ((c*st + tt)*sh + hh)*sw + ww] = w[E, c, k_t, k_h, k_w] with
-    k_t - pt = (lo_t + it)*st + tt (same for h, w); positions no kernel element maps to stay zero."""
+def _s2d_taps(w, stride, padding, dtype=torch.float32):
+    """[E, nt, nh, nw, C, st, sh, sw] in `dtype`: the conv weight scattered into the space-to-depth taps (s2d_conv_weight)."""
     E, Cin, kt, kh, kw = w.shape
     (st, sh, sw), (pt, ph, pw) = stride, padding
     lo = [_floor_div(-p_, s_) for p_, s_ in zip((pt, ph, pw), (st, sh, sw))]
     n = [_floor_div(k_ - 1 - p_, s_) - l_ + 1 for k_, p_, s_, l_ in zip((kt, kh, kw), (pt, ph, pw), (st, sh, sw), lo)]
-    W2 = torch.zeros(E, n[0], n[1], n[2], Cin, st, sh, sw, dtype=torch.float32, device=w.device)
-    wf = w.detach().float()
+    W2 = torch.zeros(E, n[0], n[1], n[2], Cin, st, sh, sw, dtype=dtype, device=w.device)
+    wf = w.detach().to(dtype)
     for a in range(kt):
         it, tt = _floor_div(a - pt, st) - lo[0], (a - pt) % st
         for bb in range(kh):
@@ -917,7 +943,24 @@ def s2d_conv_weight(w, stride, padding):
             for c in range(kw):
                 iw, ww = _floor_div(c - pw, sw) - lo[2], (c - pw) % sw
                 W2[:, it, ih, iw, :, tt, hh, ww] = wf[:, :, a, bb, c]
-    return W2.reshape(E, -1).to(torch.bfloat16).contiguous()
+    return W2
+
+
+def s2d_conv_weight(w, stride, padding):
+    """Conv3d weight [E, C, kt, kh, kw] scattered into the space-to-depth taps of csrc/patch_embed_tc.cu:
+    W2[E, ((it*nh + ih)*nw + iw) * cell + ((c*st + tt)*sh + hh)*sw + ww] = w[E, c, k_t, k_h, k_w] with
+    k_t - pt = (lo_t + it)*st + tt (same for h, w); positions no kernel element maps to stay zero."""
+    return _s2d_taps(w, stride, padding).reshape(w.shape[0], -1).to(torch.bfloat16).contiguous()
+
+
+def s2d_dgrad_weight(w, stride, padding, dtype=torch.bfloat16):
+    """Weight of the transposed stem convolution (svit_patch_embed_s2d_dgrad): [cell, ntaps * E] with
+    W''[cell, ((it*nh + ih)*nw + iw) * E + e] = W2[e, tap (nt-1-it, nh-1-ih, nw-1-iw), cell] -- s2d_conv_weight transposed,
+    tap order reversed in every dimension.  dtype float64 builds it exactly (the host-side check of the math)."""
+    taps = _s2d_taps(w, stride, padding, torch.float64 if dtype == torch.float64 else torch.float32)
+    E, nt, nh, nw = taps.shape[:4]
+    taps = taps.reshape(E, nt, nh, nw, -1).flip(1, 2, 3)
+    return taps.permute(4, 1, 2, 3, 0).reshape(taps.shape[4], -1).to(dtype).contiguous()
 
 
 def s2d_clip(clip, stride, mean=None, std=None):
@@ -967,16 +1010,80 @@ def _patch_embed_implicit(clip, w, b, cls, queries, pos_t, kernel, stride, paddi
     return x
 
 
+def d2s_clip(cells, clip_shape, stride, dtype):
+    """Inverse of s2d_clip: bf16 cells [B, Tc, Hc, Wc, C*st*sh*sw] -> clip [B, C, T, H, W] in `dtype` (fp32 / bf16)."""
+    _chk(cells, "d2s_clip")
+    cells = cells.contiguous()
+    B, Cin, T, H, W = clip_shape
+    x = torch.empty(clip_shape, dtype=dtype, device=cells.device)
+    _call("svit_d2s_clip", cells.data_ptr(), x.data_ptr(), B, Cin, T, H, W, *stride, _dt(x), _stream())
+    return x
+
+
+def patch_embed_input_grad(dx, w, clip_shape, clip_dtype, kernel, stride, padding):
+    """Gradient of the stem with respect to the clip [B, C, T, H, W] (in clip_dtype) from the sequence gradient
+    dx [B, 1 + L + Tx*O, E] (patch rows 1..L).  bf16 runs the transposed convolution on the tensor cores
+    (input_grad_s2d); fp32, and a geometry that kernel does not cover, run input_grad_col2im."""
+    Cin = clip_shape[1]
+    if dx.dtype == torch.bfloat16 and _lib.lib().svit_patch_embed_s2d_dgrad_supported(Cin, *kernel, *stride, *padding,
+                                                                                        w.shape[0]):
+        return input_grad_s2d(dx, w, clip_shape, clip_dtype, kernel, stride, padding)
+    return input_grad_col2im(dx, w, clip_shape, clip_dtype, kernel, stride, padding)
+
+
+def input_grad_s2d(dx, w, clip_shape, clip_dtype, kernel, stride, padding):
+    """bf16 dx: svit_patch_embed_s2d_dgrad reads the patch rows of dx in place (implicit GEMM over the cell grid, the
+    weight s2d_dgrad_weight cached per parameter version), then svit_d2s_clip."""
+    _chk(dx, "input_grad_s2d")
+    B, Cin, T, H, W = clip_shape
+    st, sh, sw = stride
+    E, Ntot = w.shape[0], dx.shape[1]
+    tag = ("s2d_dgrad", tuple(stride), tuple(padding))
+    wt = _cache_get(w, tag)
+    if wt is None:
+        wt = _cache_put(w, tag, s2d_dgrad_weight(w, stride, padding).to(dx.device))
+    dcells = torch.empty(B, -(-T // st), -(-H // sh), -(-W // sw), Cin * st * sh * sw, dtype=torch.bfloat16, device=dx.device)
+    _call("svit_patch_embed_s2d_dgrad", dx.data_ptr(), Ntot * E, 1, wt.data_ptr(), dcells.data_ptr(), B, Cin, T, H, W,
+          *kernel, *stride, *padding, E, _stream(), tag=f"[B{B} {T}x{H}x{W}]" if _prof is not None else None)
+    return d2s_clip(dcells, clip_shape, stride, clip_dtype)
+
+
+def input_grad_col2im(dx, w, clip_shape, clip_dtype, kernel, stride, padding):
+    """dcols = dpatch . W on svit_gemm (fp32 output; CUDA cores in the fp32 parity mode), then the svit_col2im3d gather."""
+    _chk(dx, "input_grad_col2im")
+    B, Cin, T, H, W = clip_shape
+    kt, kh, kw = kernel
+    st, sh, sw = stride
+    pt, ph, pw = padding
+    E = w.shape[0]
+    L = ((T + 2 * pt - kt) // st + 1) * ((H + 2 * ph - kh) // sh + 1) * ((W + 2 * pw - kw) // sw + 1)
+    K = Cin * kt * kh * kw
+    Kpad = (K + 63) // 64 * 64
+    dpatch = dx[:, 1:1 + L].reshape(B * L, E)  # torch view/copy glue: the patch rows, compact
+    dcols = torch.empty(B * L, Kpad, dtype=torch.float32, device=dx.device)
+    gemm(dpatch, _padded_weight(w, K, Kpad, dx.dtype), dcols, B * L, Kpad, E, E, Kpad, Kpad, 0, 0)
+    dclip = torch.empty(clip_shape, dtype=clip_dtype, device=dx.device)
+    _call("svit_col2im3d", dcols.data_ptr(), dclip.data_ptr(), B, Cin, T, H, W, *kernel, *stride, *padding, Kpad, F32,
+          _dt(dclip), _stream())
+    return dclip
+
+
 def patch_embed_tokens(clip, w, b, cls, queries, pos_t, kernel, stride, padding, dtype, mean=None, std=None):
     """[cls | conv3d(clip) patch tokens | object queries + temporal embedding].  clip: [B, C, T, H, W] (fp32 / bf16) or
     decoded uint8 frames [B, T, H, W, C].  Without autograd and in bf16 the stem is an implicit GEMM
     (csrc/patch_embed_tc.cu); with autograd (the weight gradient needs the im2col matrix) or in the fp32 parity mode it is
-    svit_im2col3d + svit_gemm."""
+    svit_im2col3d + svit_gemm.  A clip that requires grad receives its gradient (patch_embed_input_grad); when no stem
+    parameter needs one (a frozen model), bf16 keeps the implicit-GEMM forward and the backward runs the data gradient
+    alone.  uint8 frames are not differentiable."""
     kernel, stride, padding = tuple(kernel), tuple(stride), tuple(padding)
     Cin = clip.shape[-1] if clip.dtype == torch.uint8 else clip.shape[1]
     needs_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (w, b, cls, queries, pos_t))
-    if (not needs_grad and dtype == torch.bfloat16 and _state.get("implicit_patch_embed", True)
-            and _lib.lib().svit_patch_embed_s2d_supported(Cin, *kernel, *stride, *padding, w.shape[0])):
+    clip_grad = torch.is_grad_enabled() and clip.requires_grad
+    implicit = (dtype == torch.bfloat16 and _state.get("implicit_patch_embed", True)
+                and _lib.lib().svit_patch_embed_s2d_supported(Cin, *kernel, *stride, *padding, w.shape[0]))
+    if implicit and not needs_grad:
+        if clip_grad:
+            return _PatchEmbedInputGrad.apply(clip, w, b, cls, queries, pos_t, kernel, stride, padding)
         return _patch_embed_implicit(clip, w, b, cls, queries, pos_t, kernel, stride, padding, mean, std)
     if clip.dtype == torch.uint8:
         clip = normalize_u8(clip, mean, std, torch.float32 if dtype == torch.float32 else torch.bfloat16)
